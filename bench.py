@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the MGProto Gaussian-prototype hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W            (driver: torchrun for N > 1)
+    python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1)
     python bench.py --impl reference ...                     (CPU arm: the reference algorithm on host cores)
+    python bench.py ... --dump-outputs DIR                   (also write the last timed step's outputs as DIR/*.npy)
 
 Workload (BASELINE.json configs[1], named in config.workload): per GPU a batch of 256 images'
 add-on feature maps [256,128,14,14] against a 200-class x 10-prototype x 128-d diagonal-Gaussian
@@ -25,8 +26,12 @@ The backbone is outside the path (SURVEY.md section 8) and is not timed.
   reference_gpu_eager  the same-box GPU bar: the unmodified reference model.py run eagerly on cuda:0 at the same
           shapes (no_grad forward, train forward+backward, update_GMM), timed beside our stages
 
-Timing: the --steps block is repeated R >= 10 times (each bracketed by CUDA events); `value` uses the MEDIAN block,
-min/max are reported in `timing`.
+Timing: exactly --steps timed steps after the warm-up, between two CUDA events (none between the steps, which would
+add their own gaps); `value` is the images of those steps over that window.  The end-to-end leg is timed the same way.
+
+--dump-outputs DIR writes what the last timed step returned to its caller -- logits [B,C,T], loss, the feature gradient
+[B,D,H,W] -- and the mixture it left behind (means [C,K,D], weights [C,C*K]) as float32 DIR/<name>.npy (32 MB; rank 0).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +46,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: bench.py writes nothing into it
 
 CFG = dict(B=256, C=200, K=10, D=128, H=14, W=14, T=20, cap=800)
 N_ROT = 8   # distinct input batches rotated through (8 x 25.7 MB of features > the 126 MB L2)
@@ -374,6 +380,14 @@ def build_model(dev, seed=0):
     return net
 
 
+def dump_outputs(path, arrays):
+    """Write each tensor as float32 path/<name>.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def loss_fn(out, gt):
     """CE on level 0 + 0.2 * mean CE over the mining levels (ref train_and_test.py:37-41, :55) -- the library's
     fused value+gradient helper (one launch instead of the ~25 ATen launches of T separate cross_entropy calls)."""
@@ -392,8 +406,10 @@ def main():
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip the reference_gpu_eager leg")
     ap.add_argument("--no-ood", action="store_true", help="skip the configs[4] OoD-scoring throughput leg")
     ap.add_argument("--no-graph", action="store_true", help="run the device-resident leg eagerly instead of replaying a CUDA graph")
-    ap.add_argument("--reps", type=int, default=10, help="repetitions of the --steps block (median reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -431,7 +447,7 @@ def main():
         loss = loss_fn(out, gt)
         loss.backward()
         net.update_GMM()
-        return out
+        return out, loss, x.grad
 
     def barrier():
         if world > 1:
@@ -456,7 +472,7 @@ def main():
     eager_step = step
     if graphed is not None:
         def step(x, gt):                                          # noqa: F811
-            return graphed(x, gt)[0]
+            return graphed(x, gt) + (graphed.x_grad,)
 
     # ---- device-resident throughput -------------------------------------------------------
     sampler = ClockSampler(local)
@@ -466,40 +482,35 @@ def main():
         step(feats[i % N_ROT], gts[i % N_ROT])
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    R = max(10, args.reps)                        # the --steps block is repeated R times; value = median block
-    blocks = []
-    host_enq = []
     barrier()
     t_w0 = time.time()
-    launches = 0
-    for r in range(R):
-        l0 = ops.launch_count()
-        barrier()
-        e0.record()
-        t_h0 = time.perf_counter()
-        for i in range(args.steps):
-            step(feats[(r * args.steps + i) % N_ROT], gts[(r * args.steps + i) % N_ROT])
-        e1.record()
-        host_enq.append((time.perf_counter() - t_h0) * 1e3)      # host time to ENQUEUE the block (no sync inside)
-        barrier()
-        tm = torch.tensor([e0.elapsed_time(e1)], device=dev)
-        if world > 1:
-            dist.all_reduce(tm, op=dist.ReduceOp.MAX)
-        blocks.append(float(tm))
-        launches = ops.launch_count() - l0
-        if graphed is not None:                      # replays do not pass through the Python launch counter
-            launches = graphed.launches * args.steps
+    l0 = ops.launch_count()
+    e0.record()
+    t_h0 = time.perf_counter()
+    for i in range(args.steps):
+        last = step(feats[i % N_ROT], gts[i % N_ROT])
+    e1.record()
+    host_enq = (time.perf_counter() - t_h0) * 1e3                 # host time to ENQUEUE the steps (no sync inside)
+    barrier()
     t_w1 = time.time()
-    ms = statistics.median(blocks)
-    value = B * world * args.steps / (ms / 1e3)
-    timing = {"reps": R, "block_ms_median": ms, "block_ms_min": min(blocks), "block_ms_max": max(blocks),
-              "value_from": "median block of %d x %d steps, max over ranks per block" % (R, args.steps),
-              "images_per_s_min": B * world * args.steps / (max(blocks) / 1e3),
-              "images_per_s_max": B * world * args.steps / (min(blocks) / 1e3),
+    launches = ops.launch_count() - l0
+    if graphed is not None:                          # replays do not pass through the Python launch counter
+        launches = graphed.launches * args.steps
+    tm = torch.tensor([e0.elapsed_time(e1)], device=dev)
+    if world > 1:
+        dist.all_reduce(tm, op=dist.ReduceOp.MAX)
+    window_ms = float(tm)
+    ms = window_ms / args.steps
+    value = B * world * args.steps / (window_ms / 1e3)
+    timing = {"steps": args.steps, "window_ms": window_ms,
+              "value_from": "one window of %d timed steps between two CUDA events, max over ranks" % args.steps,
               "launch": launch_mode,
-              "host_enqueue_ms_median": statistics.median(host_enq),
-              "host_note": "wall time the Python / ctypes side needs to enqueue one block (no synchronisation inside): the "
-                           "step is GPU-bound while this stays below block_ms_median"}
+              "host_enqueue_ms": host_enq,
+              "host_note": "wall time the Python / ctypes side needs to enqueue the timed steps (no synchronisation inside): "
+                           "the step is GPU-bound while this stays below window_ms"}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": last[0], "loss": last[1], "x_grad": last[2],
+                                         "prototype_means": net.prototype_means, "mixture_weights": net.last_layer.weight})
 
     # ---- end to end: host buffers in, logits out ---------------------------------------------
     # every step copies its own pinned-host feature batch to the device and reads its logits back to pinned host
@@ -514,25 +525,22 @@ def main():
             if i + 1 < n:
                 feeder.stage(feats_host[(i + 1) % N_ROT])
             x_dev = feeder.acquire()
-            out = eager_step(x_dev, gts[i % N_ROT])
+            out = eager_step(x_dev, gts[i % N_ROT])[0]
             sink.put(out.detach())
             feeder.release(x_dev)
         sink.wait()
 
-    e2e_run(3)
-    e2e_blocks = []
-    for _ in range(5):
-        barrier()
-        e0.record()
-        e2e_run(args.steps)
-        e1.record()
-        barrier()
-        tm = torch.tensor([e0.elapsed_time(e1)], device=dev)
-        if world > 1:
-            dist.all_reduce(tm, op=dist.ReduceOp.MAX)
-        e2e_blocks.append(float(tm))
-    e2e_val = B * world * args.steps / (statistics.median(e2e_blocks) / 1e3)
-    timing["e2e_block_ms"] = {"median": statistics.median(e2e_blocks), "min": min(e2e_blocks), "max": max(e2e_blocks)}
+    e2e_run(W)
+    barrier()
+    e0.record()
+    e2e_run(args.steps)
+    e1.record()
+    barrier()
+    tm = torch.tensor([e0.elapsed_time(e1)], device=dev)
+    if world > 1:
+        dist.all_reduce(tm, op=dist.ReduceOp.MAX)
+    e2e_val = B * world * args.steps / (float(tm) / 1e3)
+    timing["e2e_window_ms"] = float(tm)
     clocks = sampler.stop(t_w0, t_w1) if rank == 0 else None
 
     # ---- roofline of the log-likelihood kernel (timed alone, rank 0) --------------------------
@@ -774,7 +782,7 @@ def main():
     if rank == 0:
         line = {
             "metric": "images/sec", "value": value, "unit": "images/s", "n_gpus": world, "steps": args.steps,
-            "warmup": W, "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak",
+            "warmup": W, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": _config(world),
             "pairs_per_sec": value * HW * c["C"] * c["K"],
             "e2e": {"value": e2e_val, "unit": "images/s", "h2d_bytes_per_step": B * D * HW * 4,

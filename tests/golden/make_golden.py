@@ -1,10 +1,13 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/*.npz by running the UNMODIFIED
-reference (cwangrun/MGProto, mounted read-only at /root/reference) on CPU.
+reference (cwangrun/MGProto, a checkout named by $MGPROTO_REFERENCE) on CPU.
 
-Run from the repo root in the dev container:  python tests/golden/make_golden.py
-The fixtures travel to the GPU box; the reference itself does not, and nothing in
-tests/, bench.py or smoke() reads /root/reference at run time.
+    MGPROTO_REFERENCE=<reference checkout> python tests/golden/make_golden.py
+
+The feature maps are regenerated from seeds by tests/headline_case.py (numpy) on both
+sides, so only the reference's outputs are stored; of the feature gradients and the
+normalised features, every hw_stride-th patch row and column (a fixture file stays
+under 1 MB).  Nothing in tests/, bench.py or smoke() reads the reference.
 
 Only this script imports the reference.  It touches no reference file; the two
 shims below exist because the reference hard-codes ``.cuda()`` (model.py:391, :472)
@@ -18,12 +21,14 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-REF = os.environ.get("MGPROTO_REFERENCE", "/root/reference")
-sys.path.insert(0, REF)
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
+sys.path.insert(0, os.environ["MGPROTO_REFERENCE"])
 torch.Tensor.cuda = lambda self, *a, **k: self          # CPU shim for hard-coded .cuda()
 import model as ref_model                               # noqa: E402  (the reference's model.py)
+import headline_case as HC                              # noqa: E402
 
-OUT = os.path.dirname(os.path.abspath(__file__))
+OUT = HERE
 
 
 class ResTiny(nn.Module):
@@ -58,7 +63,8 @@ def loss_fn(out, gt):
     return ce0 + 0.2 * mine                                              # train_and_test.py:37-41,55
 
 
-def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed):
+def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed, hw_stride):
+    sample = np.s_[:, :, ::hw_stride, ::hw_stride]
     g = torch.Generator().manual_seed(seed)
     m = build(C, K, D, cap, T, seed=seed)
     m.train()
@@ -71,22 +77,20 @@ def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed):
             wt[c, c * K:(c + 1) * K] = pi[c]
         m.last_layer.weight.data.copy_(wt)
     rec = dict(C=C, K=K, D=D, B=B, H=H, W=W, T=T, cap=cap, iters=iters, alpha=m.alpha, tau=m.tau,
-               num_em_loop=m.num_em_loop, lr=3e-3)
+               num_em_loop=m.num_em_loop, lr=3e-3, seed=seed, hw_stride=hw_stride)
     rec['mu0'] = m.prototype_means.detach().numpy().copy()
     rec['sigma'] = m.prototype_covs.detach().numpy().copy()
     rec['weight0'] = m.last_layer.weight.detach().numpy().copy()
 
     for it in range(iters):
-        img = torch.randn(B, 3, H, W, generator=g)
+        img = None                                                       # conv_features is pointed at x_leaf
         gt = torch.randint(0, C, (B,), generator=g)
         # keep every push within capacity: the reference's over-capacity branch draws an
         # unseeded randperm (utils/memory.py:51-53) and would make the fixture RNG-dependent
         while int(torch.bincount(gt, minlength=C).max()) * K > cap:
             gt = torch.randint(0, C, (B,), generator=g)
-        with torch.no_grad():
-            x_add, emb = m.conv_features(img)
-        # sharpen: mix some prototype directions in so top-k gaps are not all alike
-        x_leaf = (x_add * (1.0 + 0.5 * torch.rand(B, 1, H, W, generator=g))).clone().requires_grad_(True)
+        x_leaf = torch.from_numpy(HC.fixture_features(B, D, H, W, seed, it)).requires_grad_(True)
+        emb = torch.zeros(B, 8)
         orig = m.conv_features
         m.conv_features = lambda _x, _l=x_leaf, _e=emb: (_l, _e)
         mu_before = m.prototype_means.detach().numpy().copy()
@@ -96,12 +100,11 @@ def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed):
         loss.backward()
         m.conv_features = orig
         pre = 'it%d_' % it
-        rec[pre + 'x_add'] = x_leaf.detach().numpy().copy()
         rec[pre + 'gt'] = gt.numpy().copy()
         rec[pre + 'mu'] = mu_before
         rec[pre + 'weight'] = w_before
         rec[pre + 'logits'] = out.detach().numpy().copy()
-        rec[pre + 'grad_x'] = x_leaf.grad.numpy().copy()
+        rec[pre + 'grad_x'] = x_leaf.grad.numpy()[sample].copy()
         rec[pre + 'loss'] = np.float32(loss.item())
         if it == 0:
             with torch.no_grad():
@@ -118,7 +121,7 @@ def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed):
                 pf_feat, pf_dist = m.push_forward(img)
                 m.conv_features = orig
                 rec['it0_logits_nogt'] = o2.numpy().copy()
-                rec['it0_push_feat'] = pf_feat.numpy().copy()
+                rec['it0_push_feat'] = pf_feat.numpy()[sample].copy()
                 rec['it0_push_dist'] = pf_dist.numpy().copy()
         bank, mem_len = bank_arrays(m, C)
         rec[pre + 'bank'] = bank
@@ -181,8 +184,8 @@ def make_case(name, C, K, D, B, H, W, T, cap, iters, sigma_mode, pi_mode, seed):
 if __name__ == '__main__':
     torch.set_num_threads(4)
     make_case('tiny', C=4, K=3, D=8, B=8, H=4, W=4, T=5, cap=9, iters=8,
-              sigma_mode='init', pi_mode='init', seed=11)
+              sigma_mode='init', pi_mode='init', seed=11, hw_stride=1)
     make_case('small_diag', C=6, K=5, D=32, B=8, H=14, W=14, T=20, cap=20, iters=5,
-              sigma_mode='rand', pi_mode='rand', seed=12)
+              sigma_mode='rand', pi_mode='rand', seed=12, hw_stride=2)
     make_case('k10d128', C=5, K=10, D=128, B=4, H=14, W=14, T=20, cap=20, iters=4,
-              sigma_mode='init', pi_mode='init', seed=13)
+              sigma_mode='init', pi_mode='init', seed=13, hw_stride=2)

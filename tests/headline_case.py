@@ -1,9 +1,18 @@
 """Seeded inputs of the headline-shape parity cases (BASELINE.json configs[1] mixture: 200 classes x 10 prototypes,
-800-row banks; D = 128, and the D = 256 / K = 20 / K = 40 variants).  Pure numpy (PCG64 streams are stable across
-machines), shared by tests/golden/make_golden_headline.py -- which feeds them to the UNMODIFIED reference and stores
-its outputs -- and by the GPU parity tests, which regenerate them on the GPU box and feed them to the CUDA path and
-to the numpy oracle.  Test infrastructure only."""
+800-row banks; D = 128, and the D = 256 / K = 20 / K = 40 variants) and the feature maps of the small golden cases.
+Pure numpy (PCG64 streams are stable across machines), shared by tests/golden/make_golden*.py -- which feed them to
+the UNMODIFIED reference and store its outputs -- and by the tests, which regenerate them and feed them to the CUDA
+path and to the numpy oracle.  Test infrastructure only."""
 import numpy as np
+
+# headline.npz stores fixed samples of the reference's larger outputs (a fixture file stays under 1 MB); the tests take
+# the same samples of what they compute
+MU_AFTER0 = np.s_[::3, :, ::4]         # mu after the first update_GMM: every 3rd class, every 4th dimension
+MU_AFTER1 = np.s_[:, :, ::8]           # mu after the second: every class, every 8th dimension
+ADAM = np.s_[::7, :, ::4]              # Adam moments after both calls
+GRAD_X = np.s_[:, :, ::2, ::2]         # feature gradient: every other patch row and column
+LOGP_ROWS = np.s_[::194]               # rows of the unlabelled log p [B*H*W, P]
+BANK_TAIL = 16                         # newest bank rows of every class the labelled step pushed to
 
 
 def l2n(x, axis):
@@ -48,6 +57,20 @@ def head_batch(B, C, K, D, H, W, mu, seed=1, gt_fixed=()):
         if i < B:
             gt[i] = c
     return x, gt
+
+
+def fixture_features(B, D, H, W, seed, it):
+    """Add-on feature maps [B,D,H,W] of iteration `it` of the small golden cases (tests/golden/make_golden.py): what
+    the reference's 'regular' add-on layers (two 1x1 convolutions) make of a random 3-channel image -- an affine map of
+    rank 3, fixed per case -- with every patch scaled by 1 .. 1.5.  Element-wise float64 arithmetic only, so every
+    machine regenerates the same values."""
+    r = np.random.default_rng(seed)
+    a = r.standard_normal((3, D, 1, 1)) / np.sqrt(3)
+    c = 0.2 * r.standard_normal((D, 1, 1))
+    r = np.random.default_rng([seed, it])
+    img = r.standard_normal((B, 3, 1, H, W))
+    x = c + a[0] * img[:, 0] + a[1] * img[:, 1] + a[2] * img[:, 2]
+    return (x * (1.0 + 0.5 * r.random((B, 1, H, W)))).astype(np.float32)
 
 
 def bank_rows(C, K, D, cap, mu, seed=6):

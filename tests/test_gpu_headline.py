@@ -104,11 +104,11 @@ def test_headline_labelled_step_vs_reference(hl, math):
     loss.backward()
     np.testing.assert_allclose(logits.detach().cpu().numpy(), g["logits"], rtol=TOL, atol=1e-5)
     np.testing.assert_allclose(float(loss), float(g["loss"]), rtol=TOL)
-    err = normwise(x.grad.cpu().numpy(), g["grad_x"])
+    err = normwise(x.grad.cpu().numpy()[HC.GRAD_X], g["grad_x"])
     print("grad_x norm-wise error vs reference (%s): %.2e" % (math, err))
     assert err < TOL
     # per image too (an image whose gradient is small must not hide behind a large one)
-    gx, rx = x.grad.cpu().numpy(), g["grad_x"]
+    gx, rx = x.grad.cpu().numpy()[HC.GRAD_X], g["grad_x"]
     for b in range(B):
         assert normwise(gx[b], rx[b]) < 2 * TOL, b
     # indices: level 0 of every prototype, all T levels of the own class
@@ -131,7 +131,7 @@ def test_headline_labelled_step_vs_reference(hl, math):
     np.testing.assert_array_equal(net.memory_updated_cls.numpy(), g["updated_after_enqueue"])
     lin = net.queue.linear().cpu().numpy()
     for i, c in enumerate(g["touched"]):
-        np.testing.assert_allclose(lin[int(c), -32:], g["bank_tail"][i], rtol=1e-5, atol=1e-6)
+        np.testing.assert_allclose(lin[int(c), -HC.BANK_TAIL:], g["bank_tail"][i], rtol=1e-5, atol=1e-6)
 
 
 @pytest.mark.parametrize("math", ["auto", "fp32"])
@@ -148,7 +148,7 @@ def test_headline_unlabelled_and_logprob_vs_reference(hl, math):
         lp = net.compute_log_prob(xhat).reshape(-1, C * K)
     np.testing.assert_allclose(lg0.cpu().numpy(), g["logits_nogt"], rtol=TOL, atol=1e-5)
     np.testing.assert_allclose(l0.cpu().numpy(), g["logits_nogt"][:, :, 0], rtol=TOL, atol=1e-5)
-    np.testing.assert_allclose(lp[::97].cpu().numpy(), g["logp_rows"], rtol=TOL, atol=3e-5)
+    np.testing.assert_allclose(lp[HC.LOGP_ROWS].cpu().numpy(), g["logp_rows"], rtol=TOL, atol=3e-5)
     sep0 = (np.log(g["top1_val"]) - np.log(g["top2_val"])) > 1e-3
     assert (idx0.cpu().numpy()[:, :, 0][sep0] == g["top1_idx"][sep0]).all()
 
@@ -241,7 +241,8 @@ def test_headline_update_gmm_vs_reference(hl, math, path):
     g = hl
     net, outs = _run_em(g, math, path)
     (mu0, pi0), (mu1, pi1) = outs
-    e0, e1 = normwise(mu0[::3], g["mu_after0"]), normwise(mu1, g["mu_after1"])
+    mu1 = mu1[HC.MU_AFTER1]                                      # the stored samples of the reference's results
+    e0, e1 = normwise(mu0[HC.MU_AFTER0], g["mu_after0"]), normwise(mu1, g["mu_after1"])
     print("mu norm-wise error vs reference (%s, %s): %.2e / %.2e" % (math, path, e0, e1))
     assert e0 < TOL and e1 < TOL
     # per class (a class that barely moved must still be right): error relative to that class's largest |mu|
@@ -249,14 +250,14 @@ def test_headline_update_gmm_vs_reference(hl, math, path):
     s = np.abs(g["mu_after1"]).reshape(mu1.shape[0], -1).max(1)
     assert (d / s).max() < TOL
     # ... and the MOVEMENT itself (mu_after - mu_before), the quantity the update computes
-    mv_ref = g["mu_after1"].astype(np.float64) - g["mu"]
-    mv_got = mu1.astype(np.float64) - g["mu"]
+    mv_ref = g["mu_after1"].astype(np.float64) - g["mu"][HC.MU_AFTER1]
+    mv_got = mu1.astype(np.float64) - g["mu"][HC.MU_AFTER1]
     assert normwise(mv_got, mv_ref) < 2e-3, normwise(mv_got, mv_ref)
     np.testing.assert_allclose(pi0, g["pi_after0"], rtol=TOL)
     np.testing.assert_allclose(pi1, g["pi_after1"], rtol=TOL)
     st = net.prototype_optimizer.state[net.prototype_means]
     assert int(st["step"]) == int(g["adam_step"])
-    em, ev = normwise(st["exp_avg"].cpu().numpy()[::7], g["adam_m"]), normwise(st["exp_avg_sq"].cpu().numpy()[::7], g["adam_v"])
+    em, ev = normwise(st["exp_avg"].cpu().numpy()[HC.ADAM], g["adam_m"]), normwise(st["exp_avg_sq"].cpu().numpy()[HC.ADAM], g["adam_v"])
     print("Adam moments norm-wise error vs reference: %.2e / %.2e" % (em, ev))
     assert em < TOL and ev < TOL
 

@@ -37,7 +37,7 @@ def test_head_oracle_vs_reference_headline(hl):
     np.testing.assert_allclose(fw["logits"], g["logits"], rtol=1e-4, atol=1e-5)
     fw0 = O.head_forward(f64(g["x"]), f64(g["mu"]), f64(g["sg"]), f64(g["wt"]), None, T)
     np.testing.assert_allclose(fw0["logits"], g["logits_nogt"], rtol=1e-4, atol=1e-5)
-    np.testing.assert_allclose(fw0["logp"].reshape(-1, g["mu"].shape[0] * g["mu"].shape[1])[::97], g["logp_rows"],
+    np.testing.assert_allclose(fw0["logp"].reshape(-1, g["mu"].shape[0] * g["mu"].shape[1])[HC.LOGP_ROWS], g["logp_rows"],
                                rtol=1e-4, atol=1e-5)
     sep = (g["top1_val"] - g["top2_val"]) > 1e-5 * g["top1_val"]
     assert sep.mean() > 0.95
@@ -52,7 +52,7 @@ def test_head_oracle_vs_reference_headline(hl):
         p[np.arange(B), g["gt"]] -= 1.0
         gl[:, :, t] = p / B * (1.0 if t == 0 else 0.2 / (T - 1))
     gx = O.head_backward(f64(g["x"]), f64(g["mu"]), f64(g["sg"]), f64(g["wt"]), g["gt"], T, gl)
-    err = normwise(g["grad_x"], gx)
+    err = normwise(g["grad_x"], gx[HC.GRAD_X])
     print("reference fp32 grad_x vs fp64 oracle: normwise %.2e" % err)
     assert err < 1e-4
 
@@ -90,15 +90,15 @@ def test_enqueue_and_update_gmm_oracle_vs_reference_headline(hl):
     g = hl
     bank, outs, adam = _oracle_em(g, np.float64)
     np.testing.assert_array_equal(bank.mem_len, g["mem_len_after_enqueue"])
-    for i, c in enumerate(g["touched"]):                     # the 32 newest slots of every class the step pushed to
-        np.testing.assert_allclose(bank.data[c, -32:], g["bank_tail"][i], rtol=1e-5, atol=1e-6)
+    for i, c in enumerate(g["touched"]):                     # the newest slots of every class the step pushed to
+        np.testing.assert_allclose(bank.data[c, -HC.BANK_TAIL:], g["bank_tail"][i], rtol=1e-5, atol=1e-6)
     (mu0, pi0), (mu1, pi1) = outs
-    e0, e1 = normwise(g["mu_after0"], mu0[::3]), normwise(g["mu_after1"], mu1)
+    e0, e1 = normwise(g["mu_after0"], mu0[HC.MU_AFTER0]), normwise(g["mu_after1"], mu1[HC.MU_AFTER1])
     print("reference fp32 mu after update_GMM vs fp64 oracle: normwise %.2e / %.2e" % (e0, e1))
     assert e0 < 1e-4 and e1 < 1e-4
     np.testing.assert_allclose(pi0, g["pi_after0"], rtol=1e-4)
     np.testing.assert_allclose(pi1, g["pi_after1"], rtol=1e-4)
     assert adam.t == int(g["adam_step"])
-    em, ev = normwise(g["adam_m"], adam.m[::7]), normwise(g["adam_v"], adam.v[::7])
+    em, ev = normwise(g["adam_m"], adam.m[HC.ADAM]), normwise(g["adam_v"], adam.v[HC.ADAM])
     print("reference fp32 Adam moments vs fp64 oracle: normwise %.2e / %.2e" % (em, ev))
     assert em < 1e-4 and ev < 1e-4
