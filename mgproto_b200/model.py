@@ -284,11 +284,31 @@ class MGProto(nn.Module):
 
     def _hook_optimizer(self):
         """optimizer.state_dict() (checkpointing in the reference's loop) must see the Adam step count update_GMM keeps
-        on the device: fold it in right before the state is read."""
+        on the device: fold it in right before the state is read.  optimizer.load_state_dict() replaces the state:
+        fold first (a state dict that aliases the live tensors then loads the current step), and reseed the device
+        counter from the loaded step afterwards."""
         opt = self.prototype_optimizer
-        if getattr(opt, "_mgp_hooked", None) is not self and hasattr(opt, "register_state_dict_pre_hook"):
-            opt.register_state_dict_pre_hook(lambda _o: self.sync_optimizer_state())
+        if getattr(opt, "_mgp_hooked", None) is not self:
+            opt.register_state_dict_pre_hook(lambda o: self.sync_optimizer_state() if o is self.prototype_optimizer else None)
+            opt.register_load_state_dict_pre_hook(
+                lambda o, sd: self.sync_optimizer_state() if o is self.prototype_optimizer else None)
+            opt.register_load_state_dict_post_hook(lambda o: self._reseed_after_load(o))
             opt._mgp_hooked = self
+
+    def _reseed_after_load(self, opt):
+        if opt is self.prototype_optimizer and self._adam_step_dev is not None:
+            st = opt.state.get(self.prototype_means, {})
+            self._seed_adam_step(int(st["step"]) if "step" in st else 0)
+
+    def _seed_adam_step(self, step):
+        """Set the device counter to `step` (in place when it exists: a captured CUDA graph keeps reading it)."""
+        dev = self.prototype_means.device
+        if self._adam_step_dev is not None and self._adam_step_dev.device == dev:
+            self._adam_step_dev.fill_(step)
+        else:
+            self._adam_step_dev = torch.tensor([step], dtype=torch.int32, device=dev)
+        self._adam_step_seen = step
+        self._em_dirty = False
 
     def _adam_state(self):
         opt, p = self.prototype_optimizer, self.prototype_means
@@ -298,6 +318,28 @@ class MGProto(nn.Module):
             st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
             st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
         return st
+
+    def _prepare_adam(self):
+        """(param group, state) of prototype_optimizer for the fused update_GMM, or (None, None) for the generic path.
+        Creates the Adam state and (re)seeds the device step counter: host-side work that a CUDA-graph capture of
+        update_GMM must not contain, so GraphedStep calls this before capturing."""
+        group = self._adam_config()
+        if group is None:
+            return None, None
+        opt = self.prototype_optimizer
+        fresh = getattr(opt, "_mgp_hooked", None) is not self        # first call, or a new optimiser object
+        st = self._adam_state()
+        self._hook_optimizer()
+        host_step = int(st["step"])
+        if fresh or self._adam_step_dev is None or self._adam_step_dev.device != self.prototype_means.device or \
+                self._adam_step_seen is None or host_step != self._adam_step_seen:
+            # the optimiser state was stepped elsewhere: keep the steps not folded back yet -- unless the optimiser is
+            # a new object (they were the old optimiser's)
+            if not fresh and self._em_dirty and self._adam_step_dev is not None and self._adam_step_seen is not None:
+                host_step += int(self._adam_step_dev.item()) - self._adam_step_seen
+                st["step"] = torch.tensor(float(host_step)) if torch.is_tensor(st["step"]) else host_step
+            self._seed_adam_step(host_step)
+        return group, st
 
     @torch.no_grad()
     def update_GMM(self):
@@ -311,7 +353,7 @@ class MGProto(nn.Module):
         cap = q.cap_cls
         dev = self.prototype_means.device
         L = self.num_em_loop
-        group = self._adam_config()
+        group, st = self._prepare_adam()
         order = torch.empty(C, dtype=torch.int32, device=dev)
         sched = torch.empty(2, dtype=torch.int32, device=dev)
         world, rank = 1, 0
@@ -329,18 +371,6 @@ class MGProto(nn.Module):
         if group is None:
             return self._update_GMM_generic(order, sched, stats, n_split, r0, r1, world)
 
-        st = self._adam_state()
-        self._hook_optimizer()
-        host_step = int(st["step"])
-        if self._adam_step_dev is None or self._adam_step_dev.device != dev or self._adam_step_seen is None or \
-                host_step != self._adam_step_seen:
-            # first call, or the optimiser state was replaced / stepped elsewhere: (re)seed the device counter
-            if self._em_dirty and self._adam_step_dev is not None and self._adam_step_seen is not None:
-                host_step += int(self._adam_step_dev.item()) - self._adam_step_seen   # keep the steps not folded back yet
-                st["step"] = torch.tensor(float(host_step)) if torch.is_tensor(st["step"]) else host_step
-            self._adam_step_dev = torch.tensor([host_step], dtype=torch.int32, device=dev)
-            self._adam_step_seen = host_step
-            self._em_dirty = False
         lr, (b1, b2), eps = group["lr"], group["betas"], group["eps"]
         if world == 1:
             # tensor-core path (csrc/em_tc.cu): K <= 16, D in {128, 256}, sigma constant over d inside every prototype

@@ -6,7 +6,6 @@ stream through ctypes.  Nothing falls back to ATen or to the CPU.
 """
 from __future__ import annotations
 
-import collections
 import os
 
 import torch
@@ -27,21 +26,20 @@ MATH_MODES = {"fp32": MGP_MATH_FP32, "tc": MGP_MATH_TC, "auto": MGP_MATH_AUTO, "
 _iso_cache = {}
 
 
-_PROTO_OPERANDS = collections.OrderedDict()   # (mu, sigma identity + version, shape, device, stream) -> (workspace, mu, sigma)
-
-
 def sigma_is_isotropic(sigma: torch.Tensor) -> bool:
     """True if sigma is constant over the feature dim inside every prototype.  One tiny device reduction + host
-    read, cached per (storage, version): sigma never changes in the reference's training loop."""
+    read, cached per (storage, version): sigma never changes in the reference's training loop.  A write that does
+    not bump the version (through ``.data``) is not seen."""
     # ([C,K,D] and its [P,D] view are the same question: the key leaves the leading shape out)
     key = (sigma.data_ptr(), sigma._version, sigma.numel(), sigma.shape[-1], str(sigma.device))
     hit = _iso_cache.get(key)
     if hit is None:
-        hit = bool((sigma == sigma[..., :1]).all().item())
         if len(_iso_cache) >= 8:
             _iso_cache.clear()
+        # the entry keeps sigma alive: a freed block handed to a new tensor (version 0 again) would match the key
+        hit = (bool((sigma == sigma[..., :1]).all().item()), sigma)
         _iso_cache[key] = hit
-    return hit
+    return hit[0]
 
 _launches = 0          # kernels launched through this module (bench.py reports it as gpu_launches)
 
@@ -210,27 +208,15 @@ def logprob(xhat_nd, mu_pd, sigma_pd, layout=MGP_OUT_LOGP_NP, B=None, HW=None, e
         elif iso and D in (64, 128):
             m = MGP_MATH_TC_ISO
     nbytes = lib.mgp_logprob_ws_bytes(B_, HW_, P, D, m)
-    # The TMEM-resident kernel reads only prototype-side operands from the workspace (fp16 hi/lo tiles, per-prototype
-    # constants): while mu / sigma are unchanged (eval, push, OoD scoring: every batch) the pre-pass is skipped.
-    cache_key = None
-    if ws is None and m == MGP_MATH_TC_ISO and lib.mgp_logprob_ws_is_prototype_only(int(layout), P, D, m):
-        cache_key = (mu.data_ptr(), mu._version, sg.data_ptr(), sg._version, P, D, float(eps), float(eps_log),
-                     str(x.device), _stream())
-        hit = _PROTO_OPERANDS.get(cache_key)
-        if hit is not None and hit[0].numel() >= nbytes:
-            ws, m = hit[0], MGP_MATH_TC_ISO_REUSE
-            _PROTO_OPERANDS.move_to_end(cache_key)
+    # Every call rebuilds the prototype-side operands: mu can be written without a version bump (the reference's
+    # push writes through `.data`), so nothing here can tell that cached operands are still current.  A caller that
+    # keeps mu / sigma fixed passes math="tc_iso_reuse" and the workspace of a return_ws=True call instead.
     if ws is None:
         ws = torch.empty((max(16, nbytes),), device=x.device, dtype=torch.uint8)
     elif ws.numel() < nbytes:
         raise RuntimeError("mgproto_b200: workspace too small")
     check(lib.mgp_logprob_fwd(x.data_ptr(), mu.data_ptr(), sg.data_ptr(), float(eps), float(eps_log), out.data_ptr(),
                               int(layout), B_, HW_, P, D, m, ws.data_ptr(), nbytes, _stream()), "mgp_logprob_fwd")
-    if cache_key is not None and m == MGP_MATH_TC_ISO:
-        # (the entry keeps mu / sigma alive, so their addresses cannot be recycled under the key)
-        _PROTO_OPERANDS[cache_key] = (ws, mu, sg)
-        while len(_PROTO_OPERANDS) > 2:
-            _PROTO_OPERANDS.popitem(last=False)
     _count(1 if m in (MGP_MATH_TC_REUSE, MGP_MATH_TC_ISO_REUSE) else (3 if nbytes > (P * D + P) * 4 else 2))
     return (out, ws) if return_ws else out
 

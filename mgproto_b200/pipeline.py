@@ -95,6 +95,13 @@ class GraphedStep:
     kernels keep all step-dependent state (Adam step counter, bank cursors, update flags) on the device, which is what
     makes the step replayable.  Shapes are fixed; with ``torch.distributed`` initialised the all-gather of the
     multi-GPU exchange is captured with the rest (every rank must construct and call the step in lock-step).
+
+    A capture bakes in host values: prototype_optimizer's lr / betas / eps and its moment tensors, the model's tau,
+    alpha, num_em_loop, mine_T and math_mode, and the addresses of the means, sigmas and mixture weights.  Every call
+    compares them with the captured ones; after a change (an lr scheduler step, optimizer.load_state_dict, a new
+    optimiser, ...) the step is captured again before it is replayed.  A capture runs no kernels, so the step stays
+    equal to the eager one.  With torch.distributed every rank must make the same change before the same call.
+    Writes into the tensors themselves (in place, or through ``.data``) need nothing: the graph reads them.
     """
 
     def __init__(self, net, loss_fn, x_example: torch.Tensor, gt_example: torch.Tensor, warmup: int = 3):
@@ -112,13 +119,36 @@ class GraphedStep:
                 self._body()
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
-        self.graph = torch.cuda.CUDAGraph()
+        self.graph = None
+        self._capture()
+
+    def _baked(self):
+        """What a capture bakes in: (objects compared by identity, values compared by equality)."""
+        net = self.net
+        opt = net.prototype_optimizer
+        g = opt.param_groups[0] if opt is not None else {}
+        st = opt.state.get(net.prototype_means, {}) if opt is not None else {}
+        objs = (opt, st.get("exp_avg"), st.get("exp_avg_sq"))
+        vals = (float(g.get("lr", 0.0)), tuple(g.get("betas", ())), g.get("eps"), net.tau, net.alpha, net.num_em_loop,
+                net.mine_T, net.math_mode, net.prototype_means.data_ptr(), net.prototype_covs.data_ptr(),
+                net.last_layer.weight.data_ptr())
+        return objs, vals
+
+    def _capture(self):
         from . import ops
+        prepare = getattr(self.net, "_prepare_adam", None)
+        if prepare is not None and self.net.prototype_optimizer is not None:
+            prepare()                               # Adam state and step counter: eager, never inside the capture
+        if self.graph is not None:
+            self.graph.reset()
+        self.graph = torch.cuda.CUDAGraph()
         n0 = ops.launch_count()
         with torch.cuda.graph(self.graph):
             self.out, self.loss = self._body()
         self.launches = ops.launch_count() - n0      # library kernels per replay (torch's own few are not counted)
         self.x_grad = self.x.grad
+        self._captured = self._baked()
+        self._em_dirty = getattr(self.net, "_em_dirty", False)   # a replay advances the device Adam step count
 
     def close(self):
         """Release the captured graph (and its private memory pool).  With torch.distributed: call it before
@@ -135,6 +165,9 @@ class GraphedStep:
         return out, loss
 
     def __call__(self, x: torch.Tensor, gt: torch.Tensor):
+        objs, vals = self._baked()
+        if vals != self._captured[1] or any(a is not b for a, b in zip(objs, self._captured[0])):
+            self._capture()
         with torch.no_grad():
             self.x.copy_(x, non_blocking=True)
             self.gt.copy_(gt, non_blocking=True)
@@ -142,4 +175,6 @@ class GraphedStep:
         bump = getattr(self.net, "_bump_versions", None)
         if bump is not None:
             bump()
+        if self._em_dirty:
+            self.net._em_dirty = True               # sync_optimizer_state folds the replayed steps back
         return self.out, self.loss

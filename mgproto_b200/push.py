@@ -76,5 +76,7 @@ def push_prototypes(dataloader, prototype_network_parallel, class_specific=True,
             used.add(int(i))
             chosen_img[j], chosen_patch[j], chosen_dist[j] = i, arg[i, k], val[i, k]
             break
+    if (chosen_img >= 0).any():
+        torch.autograd.graph.increment_version(net.prototype_means)          # the `.data` writes above bump nothing
     log("\tpush time: \t{0}".format(time.time() - start))
     return {"image": chosen_img, "patch": chosen_patch, "distance": chosen_dist}

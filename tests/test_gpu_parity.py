@@ -367,10 +367,11 @@ def test_logprob_tmem_resident_kernel_vs_fp64(shape):
     torch.testing.assert_close(a, b, rtol=2e-5, atol=2e-5)
 
 
-def test_logprob_prototype_operands_are_cached_until_the_prototypes_change():
-    """ops.logprob (auto, isotropic sigma, [N,P]) keeps the prototype-side operands of the TMEM-resident kernel while
-    mu / sigma are unchanged (version counter) and rebuilds them after an in-place change -- including update_GMM's
-    raw-pointer writes, which bump the counters explicitly."""
+def test_logprob_prototype_operands_are_reused_only_when_passed_explicitly():
+    """ops.logprob ([N,P], isotropic sigma) skips the prototype-side pre-pass of the TMEM-resident kernel when the
+    caller hands back the workspace of an earlier call (math='tc_iso_reuse'), and rebuilds the operands on every auto
+    call -- a write through `.data` bumps no version counter, so cached operands could be stale without anything
+    noticing."""
     from mgproto_b200 import ops, _lib
     if not _lib.load().mgp_has_tensor_core_path():
         pytest.skip("library built without the tcgen05 path")
@@ -383,18 +384,25 @@ def test_logprob_prototype_operands_are_cached_until_the_prototypes_change():
     def ref(m):
         return (-0.5 * D * np.log(2 * np.pi) - sg.double().log().sum(1)[None, :]
                 - 0.5 * (((x.double()[:, None, :] - m.double()[None]) / sg.double()[None]) ** 2).sum(-1))
-    ops._PROTO_OPERANDS.clear()
     n0 = ops.launch_count()
-    a = ops.logprob(x, mu, sg, 0, math="auto")
+    a, ws = ops.logprob(x, mu, sg, 0, math="tc_iso", return_ws=True)
     n1 = ops.launch_count()
-    b = ops.logprob(x, mu, sg, 0, math="auto")                         # hit: the pre-pass is skipped
+    b = ops.logprob(x, mu, sg, 0, math="tc_iso_reuse", ws=ws)          # the pre-pass is skipped
     n2 = ops.launch_count()
-    assert len(ops._PROTO_OPERANDS) == 1 and (n2 - n1) < (n1 - n0)
+    assert (n2 - n1) < (n1 - n0)
     assert torch.equal(a, b)
     torch.testing.assert_close(a.double(), ref(mu), rtol=2e-5, atol=2e-5)
-    mu.mul_(0.5)                                                       # in place: new version, stale operands must not be used
-    c = ops.logprob(x, mu, sg, 0, math="auto")
-    torch.testing.assert_close(c.double(), ref(mu), rtol=2e-5, atol=2e-5)
+    for _ in range(2):                                                 # auto: the same kernel, the pre-pass every time
+        n3 = ops.launch_count()
+        c = ops.logprob(x, mu, sg, 0, math="auto")
+        assert ops.launch_count() - n3 == n1 - n0
+        assert torch.equal(c, a)
+    mu.data.mul_(0.5)                                                  # no version bump
+    d = ops.logprob(x, mu, sg, 0, math="auto")
+    torch.testing.assert_close(d.double(), ref(mu), rtol=2e-5, atol=2e-5)
+    mu.mul_(0.5)                                                       # in place: new version
+    e = ops.logprob(x, mu, sg, 0, math="auto")
+    torch.testing.assert_close(e.double(), ref(mu), rtol=2e-5, atol=2e-5)
     v = mu._version
     torch.autograd.graph.increment_version(mu)                         # what MGProto.update_GMM does after its kernels
     assert mu._version == v + 1
